@@ -6,6 +6,8 @@ evaluation over the ce domain, on N B200s (one process per GPU).
     python bench.py --gpus 1 --steps K --warmup W            (N>1: launched by torchrun)
     python bench.py --impl reference ...                     CPU arm: the restated reference CPU
                                                              path (oracle/) on a bounded sample
+    python bench.py ... --dump-outputs DIR                   also write a fixed sample of what the
+                                                             last timed step computed, as .npy files
 
 Prints ONE JSON line (rank 0).  metric = NTT field-ops/s: the field operations of the step's
 transforms (1.5 * N * log2 N per N-point transform, SURVEY.md §8d) divided by the time of the
@@ -27,6 +29,8 @@ LOG_N_DEFAULT = 24
 NCOLS_DEFAULT = 32
 LOG_BLOWUP = 3
 L2_BYTES = 126 << 20
+DUMP_SAMPLE = 1 << 19       # words kept per dumped array: 3 x (8 MB of halves + 4 MB of indices) stays under 64 MB
+DUMP_SEED = 0
 
 
 def field_ops(log_n, log_b, ncols):
@@ -134,6 +138,28 @@ def check_against_golden(g, root, ce_tensor, what):
         raise SystemExit(f"bench: {what}: result differs from the oracle fixture: root {got_root} vs {g['merkle_root']}, "
                          f"constraint column sha256 {ce_sha} vs {g['constraint_eval_sha256']}")
     return {"golden": "tests/golden/config3.json", "case": what, "merkle_root": True, "constraint_eval_sha256": True}
+
+
+def dump_outputs(out_dir, root, arrays):
+    """Writes a step's outputs to out_dir as float64 .npy files, so that two builds can be compared output for output:
+    merkle_root.npy holds the root's 32 bytes; for every device array of 64-bit field words (Montgomery form, as the
+    library returns them), <name>.npy holds a sample of shape (k, 2), the low and high 32-bit halves of each word (exact
+    in float64), and <name>_index.npy the flat row-major index of each sampled word.  The sample is the whole array up to
+    DUMP_SAMPLE words, else DUMP_SAMPLE positions drawn with a fixed seed: it depends only on the array's size."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "merkle_root.npy"), np.frombuffer(root, dtype=np.uint8).astype(np.float64))
+    for name, t in arrays.items():
+        flat = t.reshape(-1)
+        total = flat.numel()
+        if total <= DUMP_SAMPLE:
+            idx = np.arange(total, dtype=np.int64)
+        else:
+            idx = np.sort(np.random.default_rng(DUMP_SEED).choice(total, DUMP_SAMPLE, replace=False))
+        words = np.ascontiguousarray(flat[torch.from_numpy(idx).to(flat.device)].cpu().numpy())
+        np.save(os.path.join(out_dir, f"{name}.npy"), words.view("<u4").reshape(-1, 2).astype(np.float64))
+        np.save(os.path.join(out_dir, f"{name}_index.npy"), idx.astype(np.float64))
 
 
 # ----------------------------------------------------------------------------- CPU arm
@@ -639,6 +665,12 @@ def run_gpu(args):
     barrier()
     launches = ctx.launches - l0
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0:
+        # the last timed step's results, before the end-to-end steps below recompute them into the same buffers
+        arrays = {"constraint_eval": ce_out}
+        if world == 1:      # at N > 1 polys holds this rank's column block and lde the exchange's work buffer
+            arrays.update(polys=polys, lde=lde)
+        dump_outputs(args.dump_outputs, root, arrays)
     total_ms = t_start.elapsed_time(t_end)
     names = ["intt", "lde", "merkle", "constraint_eval"]
     phase_ms = {nm: sum(e[i].elapsed_time(e[i + 1]) for e in evs) / args.steps for i, nm in enumerate(names)}
@@ -779,7 +811,14 @@ def main():
     ap.add_argument("--no-fused-exchange", action="store_true", help="N > 1: LDE then NCCL all-to-all instead of the fused scatter")
     ap.add_argument("--no-verify", action="store_true", help="skip the comparison with the committed oracle fixtures")
     ap.add_argument("--no-extra", action="store_true", help="skip the strong-scaling, FRI-sweep and sharded-prover arms")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed to DIR/<name>.npy "
+                    "(float64; the Merkle root, the constraint column and, at N = 1, the coefficients and the LDE, each "
+                    "sampled at fixed positions to at most 2^19 words)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU arm's timed step")
     args.cpu_log_n = min(args.cpu_log_n, args.log_n)
     if args.impl == "reference":
         run_reference(args)

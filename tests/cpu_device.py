@@ -46,7 +46,11 @@ class _Event:
 
 def install():
     """idempotent; returns the ctypes handle of the CPU ABI"""
+    # the process must see no GPU even on a machine that has one: with a device visible, torch.cuda.stream() stops being a
+    # no-op and tries to make the harness's _Stream objects current.  Takes effect because CUDA is not initialised yet here.
+    os.environ["CUDA_VISIBLE_DEVICES"] = ""
     import torch
+    assert not torch.cuda.is_available(), "cpu_device.install() must run before CUDA is initialised in this process"
     from ministark_b200 import _lib, prover
     from ministark_b200 import Context
     if getattr(_lib, "_cpu_device_installed", False):
